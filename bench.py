@@ -32,6 +32,9 @@ Reference arm / cpu_baseline sample: `interact()` over the first `--ref-frames` 
 with the memory bank PRE-FILLED to the mean bank size a frame of the full clip sees (cfg2: 11.3 frames;
 the per-frame cost of the reference is linear in the bank size, so the sample's frames cost what the
 average frame of the full clip costs) — same shapes, same top-k, same per-frame work as `config`.
+`--dump-outputs DIR` writes what the timed steps hand to their caller (the u8 masks interact() returns), from
+the last headline step, as float32 .npy files (dump_outputs); inputs and weights are seeded, so the same
+arguments give the same inputs and two builds can be compared output for output.
 Timing: CUDA events on the launching stream, barrier + synchronize on both sides, max over ranks.
 Every step reads a whole clip (503 MB at cfg2) plus >200 MB of weights: inputs exceed the 126 MB L2.
 Multi-GPU: clips shard across ranks (weak scaling, no data-path collective); NCCL only for the barrier
@@ -48,6 +51,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -77,6 +81,24 @@ CONFIGS = {
 }
 # module-level views of the default configuration (tests/test_bench_cpu.py)
 H, W, K_OBJ, TOP_K = 480, 854, 1, 20
+DUMP_BYTES = 60_000_000  # --dump-outputs: at most this much on disk (a cfg2 step returns 12 x 41 MB of masks)
+
+
+def dump_outputs(out_dir, outputs, rank=0):
+    """Write the masks of one step, {(clip, interaction): u8 [T, H, W]}, as float32 `masks_clip<c>_inter<j>.npy`.
+    If they exceed DUMP_BYTES, every array keeps the same fixed, seeded sample of flat positions, written as
+    float64 `masks_sample_index.npy` (by rank 0: every rank draws the same one)."""
+    os.makedirs(out_dir, exist_ok=True)
+    numel = next(iter(outputs.values())).size
+    n = min(numel, DUMP_BYTES // (4 * len(outputs) + 8))
+    idx = None
+    if n < numel:
+        idx = np.sort(np.random.default_rng(0).choice(numel, n, replace=False))
+        if rank == 0:
+            np.save(os.path.join(out_dir, "masks_sample_index.npy"), idx.astype(np.float64))
+    for (c, j), m in sorted(outputs.items()):
+        a = m.reshape(-1)[idx] if idx is not None else m
+        np.save(os.path.join(out_dir, f"masks_clip{c:03d}_inter{j}.npy"), a.astype(np.float32))
 
 
 def _peaks():
@@ -478,6 +500,7 @@ def run_ours(args, cfgd, cfg_name):
             self.images_l, self.masks_l = [d[0] for d in data], [d[1] for d in data]
             self.checksums = [0] * L
             self.results = []
+            self.last = []  # per interaction, the masks of every clip from the latest step
             self.step_wall = []
 
         def run(self, cores, nsteps):
@@ -493,14 +516,16 @@ def run_ours(args, cfgd, cfg_name):
                     t0 = time.perf_counter()
                     for c in cores:
                         c.reset()
-                    res = None
+                    res, outs = None, []
                     for j, idx in enumerate(inter):
                         ms = self.masks_l if j == 0 else [mask2] * self.L
                         if self.L == 1:
                             res = [cores[0].interact(ms[0], idx)]
                         else:
                             res = mivos_b200.LockstepSession(cores).interact(ms, idx)
+                        outs.append(res)
                     self.results.append(res)
+                    self.last = outs
                     self.step_wall.append(time.perf_counter() - t0)  # interact() ends with a stream sync
 
         def take_checksum(self):
@@ -544,23 +569,29 @@ def run_ours(args, cfgd, cfg_name):
         del cores
         return {"ms": sharding.max_over_ranks(ms, dev), "launches": launches, "checksum": sum(per_clip), "wall": wall, "step_ms": step_ms}
 
-    def measure(act, C, L, nsteps, warm, sample_clocks=False):
-        """value (mem_profile 0) and e2e (mem_profile 1) of one (element type, lanes, lock-step) setting."""
+    def measure(act, C, L, nsteps, warm, sample_clocks=False, keep_outputs=False):
+        """value (mem_profile 0) and e2e (mem_profile 1) of one (element type, lanes, lock-step) setting.
+        keep_outputs: also return the masks of the last `value` step, {(clip, interaction): u8 [T, H, W]}."""
         lanes = [Lane(i, C, L, act) for i in range(C)]
         sampler = ClockSampler(local) if sample_clocks else None
         if sampler:
             sampler.start()
         r0 = timed_region(lanes, C, L, 0, nsteps, warm)
         clocks = sampler.stop() if sampler else None
+        outputs = {(c, j): per_clip[i] for ln in lanes for j, per_clip in enumerate(ln.last)
+                   for i, c in enumerate(ln.clips)} if keep_outputs else None
         r1 = timed_region(lanes, C, L, 1, nsteps, max(1, warm // 3))
         n = world * C * L * frames * nsteps
         out = {"value": n / (r0["ms"] / 1e3), "e2e": n / (r1["ms"] / 1e3), "ms_per_step": r0["ms"] / nsteps,
-               "e2e_ms_per_step": r1["ms"] / nsteps, "steps": nsteps, "lanes": C, "lockstep": L, "r0": r0, "r1": r1, "clocks": clocks}
+               "e2e_ms_per_step": r1["ms"] / nsteps, "steps": nsteps, "lanes": C, "lockstep": L, "r0": r0, "r1": r1, "clocks": clocks,
+               "outputs": outputs}
         return out, lanes
 
     C = max(1, args.clips_per_gpu if args.clips_per_gpu is not None else cfgd["lanes"])
     L = max(1, args.lockstep if args.lockstep is not None else cfgd["lockstep"])
-    head, lanes = measure(ACT_DTYPE, C, L, args.steps, args.warmup, sample_clocks=True)
+    head, lanes = measure(ACT_DTYPE, C, L, args.steps, args.warmup, sample_clocks=True, keep_outputs=bool(args.dump_outputs))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, head.pop("outputs"), rank)
     h2d = world * C * L * (T * 3 * nh * nw * 4 + len(inter) * (K + 1) * Hh * Ww * 4)  # whole job, like `value`
     d2h = world * C * L * len(inter) * T * Hh * Ww
 
@@ -590,7 +621,7 @@ def run_ours(args, cfgd, cfg_name):
     gc.collect(); torch.cuda.empty_cache()
 
     # ---------------- the same metric through ONE InferenceCore.interact, and on the fp32-comparable path
-    xs = max(2, min(args.steps, args.extra_steps))
+    xs = max(1, min(args.steps, args.extra_steps))
     single = tf32 = None
     if not args.skip_extras:
         if C * L > 1:
@@ -674,6 +705,8 @@ def main():
     ap.add_argument("--skip-extras", action="store_true", help="no single-session / other-dtype measurements")
     ap.add_argument("--skip-cuda-eager", action="store_true", help="no PyTorch-eager CUDA comparator")
     ap.add_argument("--skip-roofline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the masks the last timed step returned as DIR/<name>.npy (float32; a fixed sample if large)")
     ap.add_argument("--act", default=os.environ.get("MIVOS_ACT_DTYPE", DEFAULT_ACT), choices=["tf32", "fp16"],
                     help="convolution operand / activation type of the headline measurement (fp16 = the reference GUI's autocast "
                          "precision; the other type is measured beside it)")
@@ -683,6 +716,8 @@ def main():
                     help="clips each lane advances in lock-step as ONE batch through the conv layers (mivos_b200.LockstepSession); "
                          "1 = off; default per configuration (cfg2: 3 lanes x 4 clips)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     global ACT_DTYPE
     ACT_DTYPE = torch.float16 if args.act == "fp16" else torch.float32
     cfgd = dict(CONFIGS[args.config])

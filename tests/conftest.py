@@ -21,6 +21,17 @@ def _no_grad():
     yield
 
 
+@pytest.fixture(scope="session", autouse=True)
+def _golden_threads():
+    """The thread count tests/golden/ was generated with, whatever the host's core count: the CPU oracle then
+    reproduces the goldens' bits (oracle.GOLDEN_THREADS)."""
+    from oracle import GOLDEN_THREADS
+    n = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    yield
+    torch.set_num_threads(n)
+
+
 @pytest.fixture(scope="session")
 def prop_sd():
     from oracle import weights

@@ -77,6 +77,30 @@ def test_cpu_sample_is_the_configured_workload(monkeypatch):
     assert m4.shape == (5, 64, 96)
 
 
+def test_dump_outputs_whole_and_sampled(tmp_path, monkeypatch):
+    """--dump-outputs: float32 masks per (clip, interaction), whole when they fit DUMP_BYTES, otherwise the
+    same seeded sample of positions in every array, identical from run to run."""
+    import bench
+    import numpy as np
+    rng = np.random.default_rng(1)
+    outs = {(c, j): rng.integers(0, 3, (5, 8, 12), dtype=np.uint8) for c in range(3) for j in range(2)}
+    bench.dump_outputs(str(tmp_path / "whole"), outs)
+    assert not (tmp_path / "whole" / "masks_sample_index.npy").exists()
+    for (c, j), m in outs.items():
+        a = np.load(tmp_path / "whole" / f"masks_clip{c:03d}_inter{j}.npy")
+        assert a.dtype == np.float32 and np.array_equal(a, m)
+    monkeypatch.setattr(bench, "DUMP_BYTES", 100 * (4 * len(outs) + 8))  # room for 100 elements per array
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), outs)
+    idx = np.load(tmp_path / "a" / "masks_sample_index.npy")
+    assert idx.dtype == np.float64 and idx.shape == (100,) and len(set(idx.tolist())) == 100
+    assert np.array_equal(idx, np.load(tmp_path / "b" / "masks_sample_index.npy"))
+    for (c, j), m in outs.items():
+        a = np.load(tmp_path / "a" / f"masks_clip{c:03d}_inter{j}.npy")
+        assert a.dtype == np.float32 and np.array_equal(a, m.reshape(-1)[idx.astype(np.int64)])
+    assert sum(f.stat().st_size - 128 for f in (tmp_path / "a").iterdir()) <= bench.DUMP_BYTES  # (npy headers: 128 B)
+
+
 def test_propagated_frames_and_workload_config():
     import bench
     assert bench.propagated_frames(101, (0,)) == 100

@@ -1,132 +1,103 @@
-"""CPU, build container only: the oracle against the UNMODIFIED reference run LIVE (imported from
-/root/reference through oracle/refshim.py) on inputs and seeds that are NOT the committed fixtures — the
-oracle is pinned to the reference itself, not only to vectors generated once.  Skipped where the
-reference tree is absent (the GPU box has none; nothing under `-m gpu`, smoke() or bench.py reads it)."""
+"""CPU: the oracle against what the UNMODIFIED reference computed on inputs and seeds that are NOT the other
+fixtures — the oracle is pinned to the reference on a second, independent set of inputs.  The reference's
+outputs are tests/golden/reference_live.npz (oracle/gen_golden_live.py, which also checked the oracle
+bit for bit against the reference when it wrote them; large outputs are kept as a fixed sample of
+elements, `gen_golden_live.sample`).  Integer outputs must match exactly; floating-point ones to TOL of
+their largest magnitude, which only absorbs a different CPU's oneDNN/MKL kernel choice."""
 import numpy as np
 import pytest
 import torch
 
-from oracle import refshim
+from oracle import gen_golden_live as L
 
-pytestmark = pytest.mark.skipif(not refshim.available(), reason="/root/reference is only present in the build container")
+TOL = 1e-5
 
 
 @pytest.fixture(scope="module")
-def ref():
-    r = refshim.load_reference()
-    yield r
-    r._restore()
+def ref(golden):
+    return golden("reference_live.npz")
+
+
+def _close(ours, ref, key, tol=TOL):
+    """`ours` (whole) against the reference's output `key` (whole or sampled) of the golden file."""
+    assert tuple(ours.shape) == tuple(ref[f"{key}_shape"])
+    ours, want = L.sample(ours).astype(np.float64), ref[key].astype(np.float64)
+    assert float(np.abs(ours - want).max()) <= tol * max(1.0, float(np.abs(want).max())), float(np.abs(ours - want).max())
 
 
 def test_propagation_ops_live(ref, prop_sd, fuse_sd):
-    from oracle import stm_oracle as O, weights as Wt
-    net = ref.build_prop(prop_sd, top_k=20)
-    fuse = ref.build_fusion(fuse_sd)
-    images, mask = Wt.synthetic_clip(3, 64, 96, 3, seed=2024)  # three objects: the "others" channel sums two masks
+    from oracle import stm_oracle as O
+    images, mask = L.ops_inputs()
     frame = images[:, 1]
-    for a, b in zip(O.get_query_values(prop_sd, frame), net.get_query_values(frame)):
-        assert torch.equal(a, b)
-    mk, mv = net.memorize(frame, mask[1:])
-    ok, ov = O.memorize(prop_sd, frame, mask[1:])
-    assert torch.equal(ok, mk) and torch.equal(ov, mv)
-    qv = net.get_query_values(images[:, 2])
-    seg = net.segment_with_query(mk, mv, *qv)
-    assert torch.equal(O.segment_with_query(prop_sd, mk, mv, *qv, top_k=20), seg)
-    agg = ref.aggregate_wbg(seg, keep_bg=True)
-    assert torch.equal(O.aggregate_wbg(seg, keep_bg=True), agg)
+    for name, a in zip(("f16", "f8", "f4", "k16", "v16"), O.get_query_values(prop_sd, frame)):
+        _close(a, ref, f"ops_{name}")
+    mk, mv = O.memorize(prop_sd, frame, mask[1:])
+    _close(mk, ref, "ops_mem_k")
+    _close(mv, ref, "ops_mem_v")
+    qv = O.get_query_values(prop_sd, images[:, 2])
+    seg = O.segment_with_query(prop_sd, mk, mv, *qv, top_k=20)
+    _close(seg, ref, "ops_seg")
+    agg = O.aggregate_wbg(seg, keep_bg=True)
+    _close(agg, ref, "ops_agg")
     assert float(np.abs(O.aggregate_wbg_f64(seg.numpy(), keep_bg=True) - agg.numpy()).max()) <= 5e-7
     pos, neg = (mask[1:2] - seg[0:1]).clamp(0, 1), (seg[0:1] - mask[1:2]).clamp(0, 1)
-    at = net.get_attention(mk[0:1], pos, neg, qv[3])
-    assert torch.equal(O.get_attention(None, mk[0:1], pos, neg, qv[3]), at)
+    at = O.get_attention(None, mk[0:1], pos, neg, qv[3])
+    _close(at, ref, "ops_attn")
     assert float(np.abs(O.get_attention_f64(mk[0:1].numpy(), pos.numpy(), neg.numpy(), qv[3].numpy()) - at.numpy()).max()) <= 2e-6
     dist = torch.tensor([[0.25, 0.75]])
-    fu = fuse(images[:, 2], seg[0:1], agg[1:2], at, dist)
-    assert torch.equal(O.fusion_net(fuse_sd, images[:, 2], seg[0:1], agg[1:2], at, dist), fu)
+    _close(O.fusion_net(fuse_sd, images[:, 2], seg[0:1], agg[1:2], at, dist), ref, "ops_fuse")
 
 
 def test_inference_core_live(ref, prop_sd, fuse_sd):
     """Whole interact() runs, two interactions (the second one fuses): bank trace is not observable in the
-    reference, so probabilities and masks are compared — identical."""
-    from oracle import stm_oracle as O, weights as Wt
-    images, mask = Wt.synthetic_clip(7, 64, 88, 2, seed=77)  # 88 -> padded to 96
-    net, fuse = ref.build_prop(prop_sd, top_k=20), ref.build_fusion(fuse_sd)
-    rc = ref.InferenceCore(net, fuse, images, 2, mem_profile=0, mem_freq=2, device="cpu")
+    reference, so probabilities and masks are compared."""
+    from oracle import stm_oracle as O
+    images, inters = L.core_inputs()
     oc = O.OracleInferenceCore(prop_sd, fuse_sd, images, 2, mem_freq=2, top_k=20)
-    for m, idx in ((mask, 1), (mask.flip(-1).contiguous(), 6)):
-        rm = rc.interact(m, idx)
+    for j, (m, idx) in enumerate(inters, 1):
         om = oc.interact(m, idx)
-        assert (rm == om).all() and rm.shape == (7, 64, 88)
-        assert torch.equal(rc.prob, oc.prob)
-    assert torch.equal(rc.certain_mem_k, oc.certain_mem_k)
+        assert (om == ref[f"core_masks{j}"]).all() and om.shape == (7, 64, 88)
+        _close(oc.prob, ref, f"core_prob{j}")
+    _close(oc.certain_mem_k, ref, "core_certain_k")
 
 
 def test_s2m_live(ref):
     from oracle import s2m_oracle as S, weights as Wt
     sd = Wt.make_s2m_state_dict()
-    with refshim.reference_on_path():
-        from interact.s2m_controller import S2MController
-        from model.s2m.s2m_network import deeplabv3plus_resnet50 as S2M
-        net = S2M().eval()
-        net.load_state_dict(sd, strict=True)
-        x = torch.randn((2, 6, 64, 80), generator=torch.Generator().manual_seed(5))
-        assert torch.equal(S.s2m_forward(sd, x), net(x))
-        image = torch.randn((1, 3, 64, 80), generator=torch.Generator().manual_seed(6))
-        prev = torch.zeros((1, 64, 80), dtype=torch.int64)
-        prev[:, 10:30, 10:40] = 1
-        scr = np.full((60, 75), 255, dtype=np.uint8)  # unpadded: the controller pads the scribble maps
-        scr[20:22, 5:50] = 1
-        scr[40:42, 30:70] = 0
-        ctrl = S2MController(net, 1, ignore_class=255, device="cpu")
-        assert torch.equal(S.s2m_controller_interact(sd, image, prev, scr, 1), ctrl.interact(image, prev, scr))
+    x, image, prev, scr = L.s2m_inputs()
+    _close(S.s2m_forward(sd, x), ref, "s2m_logits")
+    _close(S.s2m_controller_interact(sd, image, prev, scr, 1), ref, "s2m_controller")
 
 
-def test_egress_live():
+def test_egress_live(ref):
     from oracle import egress_oracle as EO
-    from oracle.gen_golden_egress import load_reference_utils
-    iu, pal = load_reference_utils()
-    assert np.array_equal(pal.pal_color_map(), EO.color_map())
-    rng = np.random.default_rng(9)
-    image = rng.integers(0, 256, size=(40, 52, 3), dtype=np.uint8)
-    mask = rng.integers(0, 7, size=(40, 52), dtype=np.uint8) * (rng.random((40, 52)) > 0.6)
-    mask = mask.astype(np.uint8)
-    for alpha in (0.5, 0.37):
-        assert np.array_equal(iu.overlay_davis(image, mask, alpha), EO.overlay_davis(image, mask, alpha))
-        assert np.array_equal(iu.overlay_davis_fade(image, mask, alpha), EO.overlay_davis(image, mask, alpha, fade=True))
+    assert np.array_equal(ref["egress_palette"], EO.color_map())
+    image, mask = L.egress_inputs()
+    for alpha in L.EGRESS_ALPHAS:
+        a = int(round(alpha * 100))
+        assert np.array_equal(ref[f"egress_overlay_a{a}"], EO.overlay_davis(image, mask, alpha))
+        assert np.array_equal(ref[f"egress_fade_a{a}"], EO.overlay_davis(image, mask, alpha, fade=True))
 
 
 def test_fusion_generator_flow_live(ref, prop_sd):
     """SURVEY §8f-1: the client flow restated in tests/test_gpu_clients.py (what the GPU test drives our
-    PropagationNetwork through) equals the reference's real FusionGenerator class."""
+    PropagationNetwork through) equals what the reference's real FusionGenerator class returned."""
     import types
-    from oracle import stm_oracle as O, weights as Wt
+    from oracle import stm_oracle as O
     from test_gpu_clients import fusion_generator_flow
-    images, mask = Wt.synthetic_clip(5, 128, 168, 2, seed=31)
-    soft = mask[1:] * 0.8 + 0.05
-    net = ref.build_prop(prop_sd, top_k=50)
-    with refshim.reference_on_path():
-        import importlib
-        FusionGenerator = importlib.import_module("generation.fusion_generator").FusionGenerator
-        import sys
-        for k in [k for k in sys.modules if k == "generation" or k.startswith("generation.")]:
-            sys.modules.pop(k)
-    gen = FusionGenerator(net, images, mem_freq=2)
-    gen.reset(2)
-    ref_prob = gen.interact_mask(soft, 2, 0, 4)  # [K+1, T, h, w], unpadded
+    images, soft = L.fusion_generator_inputs()
     api = types.SimpleNamespace(pad_divide_by=O.pad_divide_by, aggregate_wbg=O.aggregate_wbg,
                                 memorize=lambda f, m: O.memorize(prop_sd, f, m),
                                 get_query_values=lambda f: O.get_query_values(prop_sd, f),
                                 segment_with_query=lambda *a: O.segment_with_query(prop_sd, *a, top_k=50))
     prob = fusion_generator_flow(api, images, soft, 2, 0, 4, mem_freq=2)  # [K+1, T, 1, nh, nw], padded 168 -> 176
-    assert torch.equal(prob[:, :, 0, :, 4:-4], ref_prob)
+    assert prob.shape == (3, 5, 1, 128, 176)
+    _close(prob[:, :, 0, :, 4:-4].contiguous(), ref, "fusion_generator_prob")  # the reference returns it unpadded
 
 
 def test_attention_read_network_live(ref, prop_sd):
     """SURVEY §8f-2: AttentionReadNetwork.forward (model/attn_network.py:48-80) on a fresh batch."""
     from oracle import stm_oracle as O
-    net = ref.build_attn(prop_sd)
-    g = torch.Generator().manual_seed(123)
-    image, query = torch.randn((1, 3, 48, 80), generator=g), torch.randn((1, 3, 48, 80), generator=g)
-    m11, m21, m12, m22 = (torch.rand((1, 1, 48, 80), generator=g) for _ in range(4))
-    a1, a2 = net(image, m11, m21, m12, m22, query)
-    o1, o2 = O.attention_read_network(prop_sd, image, m11, m21, m12, m22, query)
-    assert torch.equal(o1, a1) and torch.equal(o2, a2)
+    o1, o2 = O.attention_read_network(prop_sd, *L.attn_inputs())
+    _close(o1, ref, "attn1")
+    _close(o2, ref, "attn2")
